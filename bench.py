@@ -12,6 +12,7 @@ weights (no checkpoints offline), fp16 storage + fp32 accumulation like the refe
     python bench.py --impl torch-cuda ...                    the same algorithm through stock PyTorch CUDA ops on this GPU
     python bench.py --views 4 | --res 1024 --dtype bf16 | --views 64 (8 GPUs) | --shading splitsum    BASELINE configs 2 / 3 / 4 / a5
     python bench.py --gpus 2 --check                         + gradient identity of the sharded step vs one process
+    python bench.py --dump-outputs DIR                       + what the last timed step computed, as DIR/<name>.npy
 """
 import argparse
 import json
@@ -162,6 +163,9 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     device = f"cuda:{local}"
+    # the step's device-side draws (jitter, MC samples, timesteps, noise, VAE posterior) come from the default CUDA
+    # generator, which PyTorch otherwise seeds at random per process: fixed here so a run's inputs repeat; one stream per rank
+    torch.cuda.manual_seed(rank)
     if world > 1:
         # NCCL_DEBUG is left exactly as the launcher set it (its banner goes to stderr with everything else, see main())
         dist.init_process_group("nccl", device_id=torch.device(device))
@@ -241,7 +245,7 @@ def run_ours(args):
         out = sysm.training_step_fused(b, global_views=V, total_pn_global=tot_pn)
         if mode != "device":
             return float(out["loss"])      # D2H read of the step's result
-        return out["loss"]
+        return out
 
     def timed(n_warm, n_steps, mode):
         for _ in range(n_warm):
@@ -258,7 +262,10 @@ def run_ours(args):
         ev[0].record()
         host, seg0 = [time.perf_counter()], torch.cuda.memory_stats().get("num_device_alloc", 0)
         for i in range(n_steps):
-            step(mode)
+            if i + 1 < n_steps:
+                step(mode)
+            else:
+                last = step(mode)      # only the final result is held: earlier steps free theirs as soon as they return
             ev[i + 1].record()
             host.append(time.perf_counter())
         torch.cuda.synchronize()
@@ -275,13 +282,17 @@ def run_ours(args):
                   "steps_over_1p5x_median": sum(1 for x in per if x > 1.5 * per[len(per) // 2]),
                   "slowest_step": {"index": worst, "host_ms": (host[worst + 1] - host[worst]) * 1e3,
                                    "cudaMalloc_calls_in_region": torch.cuda.memory_stats().get("num_device_alloc", 0) - seg0}}
-        return float(ms) / n_steps, (l1 - l0) // n_steps, spread
+        return float(ms) / n_steps, (l1 - l0) // n_steps, spread, last
 
     sampler = ClockSampler(local) if rank == 0 else None
-    ms_step, launches, spread = timed(args.warmup, args.steps, "device")
+    ms_step, launches, spread, last = timed(args.warmup, args.steps, "device")
+    if args.dump_outputs and rank == 0:
+        # before the profiled and e2e steps below: they overwrite the captured graphs' canvas that comp_rgb views
+        dump_outputs(args.dump_outputs, last)
+    del last
     # section split (one extra profiled step, outside the timed region)
     sec = sysm.profile_step(lambda: make_batch("device")[:2], V) if hasattr(sysm, "profile_step") else {}
-    ms_e2e, _, spread_e2e = timed(max(1, args.warmup // 2), args.steps, "e2e")
+    ms_e2e, _, spread_e2e, _ = timed(max(1, args.warmup // 2), args.steps, "e2e")
     parity = gradient_identity_check(sysm, make_batch, cam_dev, V, world, rank, device) if args.check else None
     clocks = sampler.stop() if sampler else None
     if rank != 0:
@@ -722,6 +733,26 @@ def run_reference(args):
     emit(out)
 
 
+DUMP_MAX_ELEMS = 1 << 23        # 32 MB of float32: comp_rgb of the default workload (8 x 512 x 512 x 3) fits whole
+
+
+def dump_outputs(out_dir, out):
+    """--dump-outputs: what one training step hands its caller -- every entry of training_step_fused's result (the losses,
+    the logged norms, comp_rgb) -- as float32 DIR/<name>.npy.  A larger comp_rgb (more views, higher resolution) is written
+    as a fixed sample of its flattened values (seeded, sorted indices), so two builds of the project compare element for
+    element.  The parameters after Adam are left out: with eps = 1e-15 a near-zero gradient entry moves by +-lr whatever
+    its sign, so they differ between two runs of the same build far more than any output does."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 _RESULT_FD = None
 
 
@@ -754,7 +785,12 @@ def main():
     ap.add_argument("--no-pdl", action="store_true", help="disable programmatic dependent launch of the dense kernels")
     ap.add_argument("--no-gc-freeze", action="store_true", help="A/B: leave Python's full collections inside the timed region")
     ap.add_argument("--no-balance", action="store_true", help="multi-GPU: every rank shades only its own views")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     # stdout carries exactly one JSON line: libraries that write to fd 1 (NCCL's version banner, nvcc/ninja chatter)
     # are sent to stderr for the whole run and the result line is written to the saved descriptor.
     global _RESULT_FD

@@ -4,7 +4,7 @@ pytorch_lightning / omegaconf / diffusers / nvdiffrast are absent on the build a
 cannot be imported there.  This stub restates only the INTERFACE the five plugins of dreammat_b200.threestudio_plugin
 touch (registry, BaseObject / BaseModule construction protocol, Updateable walk, BaseLift3DSystem wiring, parse_optimizer)
 so that `threestudio.find("dreammat-system")(cfg)` can be driven end to end.  tests/test_plugin_registry.py pins its
-behaviour against the reference's own code (executed from /root/reference by AST) where that tree is present.
+behaviour against the reference's own code (the event log recorded in tests/golden/threestudio_protocol.json).
 
 Registry: threestudio/__init__.py:1-13 of the reference (module-level dict, last writer wins).
 """

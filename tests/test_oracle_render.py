@@ -3,13 +3,12 @@ import math
 import os
 
 import numpy as np
-import pytest
 import torch
 
 from oracle import render as O
 from tests._fixtures import make_scene, rel_err
 
-REF = "/root/reference/threestudio_dreammat"
+ASSETS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "splitsum_assets.pt")
 
 
 def test_bvh_matches_brute_force():
@@ -65,11 +64,11 @@ def test_mc_shading_white_furnace_and_grad():
     assert torch.isfinite(g).all() and float(g.abs().sum()) > 0
 
 
-@pytest.mark.skipif(not os.path.exists(REF + "/load/lights/bsdf_256_256.bin"), reason="reference fixture absent")
 def test_fg_lut_fixture_is_the_split_sum_brdf_integral():
     """Pins fg_lookup's axis convention (u = N.V -> W, v = roughness -> H) against the only golden
-    data the reference holds for this path: the LUT must equal Karis' split-sum DFG integral."""
-    lut = torch.from_numpy(np.fromfile(REF + "/load/lights/bsdf_256_256.bin", dtype=np.float32).reshape(256, 256, 2))
+    data the reference holds for this path: the LUT must equal Karis' split-sum DFG integral.
+    The reference's load/lights/bsdf_256_256.bin is stored whole in tests/golden/splitsum_assets.pt."""
+    lut = torch.load(ASSETS)["fg_lut"][0]
 
     def dfg(ndv, rough, n=4096):
         a = rough * rough

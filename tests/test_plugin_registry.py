@@ -1,15 +1,15 @@
 """Drop-in boundary (SURVEY.md section 8b), host side, no GPU.
 
 1. The stub `threestudio` package under tests/stub_threestudio (the reference package cannot be imported here:
-   pytorch_lightning / omegaconf / nvdiffrast ... are absent) is PINNED against the reference's own code: the registry
-   functions and the Updateable / BaseObject / BaseModule classes are lifted out of /root/reference by AST (nothing is
-   copied into the repo), executed, and driven through the same scenario as the stub.
+   pytorch_lightning / omegaconf / nvdiffrast ... are absent) is PINNED against the reference's own code: the event log
+   the reference's registry functions and Updateable / BaseObject / BaseModule classes produce for one scenario is
+   recorded in tests/golden/threestudio_protocol.json, and the stub must produce the same log.
 2. With the stub importable, `import dreammat_b200.threestudio_plugin` must re-register the five names of
    configs/dreammat.yaml:28-97, construct through `cls(cfg)` -> `configure()`, reject unknown config keys, and
    produce / accept the reference's state-dict keys with strict=True.
 """
-import ast
 import dataclasses
+import json
 import os
 import sys
 import textwrap
@@ -19,7 +19,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 STUB = os.path.join(ROOT, "tests", "stub_threestudio")
-REF = "/root/reference/threestudio_dreammat/threestudio"
+PROTOCOL = os.path.join(ROOT, "tests", "golden", "threestudio_protocol.json")
 
 FIVE = ["dreammat-system", "dreammat-mesh", "dreammat-material", "raytracing-renderer", "stable-diffusion-dreammat-guidance"]
 
@@ -56,31 +56,6 @@ def stub_on_path():
         sys.path.remove(STUB)
         for m in [k for k in sys.modules if k == "threestudio" or k.startswith("threestudio.") or k == "dreammat_b200.threestudio_plugin"]:
             del sys.modules[m]
-
-
-def _lift(path, names):
-    """source of the named top-level functions / classes of a reference file, annotations stripped"""
-    tree = ast.parse(open(path).read())
-
-    class Strip(ast.NodeTransformer):
-        def visit_FunctionDef(self, node):
-            self.generic_visit(node)
-            node.returns = None
-            for a in node.args.args + node.args.kwonlyargs:
-                a.annotation = None
-            return node
-
-        def visit_AnnAssign(self, node):
-            if node.value is None:
-                return None
-            return ast.copy_location(ast.Assign(targets=[node.target], value=node.value), node)
-
-    out = []
-    for node in tree.body:
-        if isinstance(node, (ast.FunctionDef, ast.ClassDef)) and node.name in names:
-            out.append(ast.unparse(ast.fix_missing_locations(Strip().visit(node))))
-    assert len(out) == len(names), (path, names)
-    return "\n\n".join(out)
 
 
 def _scenario(ns):
@@ -141,23 +116,22 @@ def _scenario(ns):
     return log
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 def test_stub_matches_reference_protocol(stub_on_path):
+    """The reference's own register / find / Updateable / BaseObject / BaseModule, driven through `_scenario` with its two
+    un-importable helpers injected (parse_structured without omegaconf, get_device as in the stub), produced the log in
+    tests/golden/threestudio_protocol.json; the stub must produce the same one."""
     import threestudio as stub
     from threestudio.utils import base as sbase
+    from threestudio.utils.misc import get_device
     stub_ns = dict(register=stub.register, find=stub.find, BaseObject=sbase.BaseObject, BaseModule=sbase.BaseModule,
                    Updateable=sbase.Updateable)
-    # the reference's own code, lifted by AST; its two un-importable helpers are injected: parse_structured without
-    # omegaconf (= the dataclass instance), get_device as in the stub, load_module_weights unused here
-    from threestudio.utils.config import parse_structured
-    from threestudio.utils.misc import get_device
-    ref_ns = {"__modules__": {}, "dataclass": dataclasses.dataclass, "torch": torch, "nn": torch.nn, "parse_structured": parse_structured,
-              "get_device": get_device, "load_module_weights": None}
-    exec(_lift(os.path.join(REF, "__init__.py"), ["register", "find"]), ref_ns)
-    exec(_lift(os.path.join(REF, "utils", "base.py"), ["Updateable", "BaseObject", "BaseModule"]), ref_ns)
-    a, b = _scenario(stub_ns), _scenario(ref_ns)
-    assert a == b, "\n".join(f"{x}   |   {y}" for x, y in zip(a, b))
-    assert ("unknown", "raises") in a and ("find", "B") in a
+    with open(PROTOCOL) as f:
+        want = json.load(f)["log"]
+    # both sides asked the same injected get_device(): the recorded entry holds no device name
+    want = [[e[0], str(get_device()), *e[2:]] if e[0] == "device" else e for e in want]
+    a = json.loads(json.dumps(_scenario(stub_ns)))      # tuples -> lists, as recorded
+    assert a == want, "\n".join(f"{x}   |   {y}" for x, y in zip(a, want))
+    assert ["unknown", "raises"] in a and ["find", "B"] in a
 
 
 def _write_obj(path):
