@@ -100,6 +100,10 @@ SIGNATURES = {
     "dm_hp_split": (C.c_int, [P, I64, C.c_int, I64, C.c_int, P, P]),
     "dm_hp_epilogue": (C.c_int, [P, I64, C.c_int, I64, P, P, I64, I64, P]),
     "dm_conv2d": (C.c_int, [C.c_int, P] + [C.c_int] * 4 + [P] + [C.c_int] * 7 + [P, I64, P, C.c_int, P]),
+    "dm_uv_raster": (C.c_int, [P, P, I64, C.c_int, P, P, P, P]),
+    "dm_texel_positions": (C.c_int, [P, I64, P, P, P, P, P, P]),
+    "dm_material_export": (C.c_int, [P, P, I64, P, P, P, P, P, P]),
+    "dm_seam_fill": (C.c_int, [P, C.c_int] + [P] * 9),
 }
 
 

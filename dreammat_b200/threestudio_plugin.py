@@ -1,4 +1,4 @@
-"""Drop-in plugin layer: registers the five hot-path plugins under the reference's registry names.
+"""Drop-in plugin layer: registers the five hot-path plugins and the mesh exporter under the reference's registry names.
 
     import threestudio                      # the reference package (threestudio_dreammat/threestudio)
     import dreammat_b200.threestudio_plugin # re-registers the names below; last writer wins (threestudio/__init__.py:4-13)
@@ -8,11 +8,13 @@
     dreammat-material                    models/materials/dreammat_material.py:346 -> DreamMatMaterial
     raytracing-renderer                  models/renderers/raytracing_renderer.py:86 -> RaytraceRender
     stable-diffusion-dreammat-guidance   models/guidance/dreammat_guidance.py:44 -> StableDiffusionLightGuidance
+    mesh-exporter                        models/exporters/mesh_exporter.py    -> MeshExporter (texbake.py)
 
 Every class keeps the reference's construction protocol -- `cls(cfg, *args, **kwargs)` -> `parse_structured(Config, cfg)`
 -> `configure(*args, **kwargs)` (utils/base.py:70-118; the system: systems/base.py:35-50) -- its Config field names /
 defaults, call signatures, output keys and state-dict keys, so `launch.py` with `configs/dreammat.yaml` drives it
-unchanged: the data module, prompt processor, background, Lightning trainer, logging and exporters stay the reference's.
+unchanged: the data module, prompt processor, background, Lightning trainer and logging stay the reference's; the exporter's
+output goes through the host's own `save_obj`.
 
 The classes derive from threestudio's own bases (BaseModule / BaseObject / BaseLift3DSystem): `isinstance(x, Updateable)`
 keeps working, so the system's per-step `do_update_step` walk reaches `guidance.update_step` exactly as before.
@@ -29,6 +31,7 @@ import torch
 import torch.nn as nn
 
 import threestudio
+from threestudio.models.exporters.base import Exporter, ExporterOutput
 from threestudio.systems.base import BaseLift3DSystem
 from threestudio.utils.base import BaseModule, BaseObject
 
@@ -36,6 +39,7 @@ from . import guidance as _G
 from . import render_ops as R
 from . import scene as _S
 from . import system as _Y
+from . import texbake as _T
 from . import weights as _W
 
 
@@ -426,3 +430,67 @@ class DreamMat(BaseLift3DSystem):
     def on_test_epoch_end(self):
         """systems/dreammat.py:298-300"""
         self.save_gif("it" + str(self.true_global_step) + "-test/view", fps=30)
+
+
+# ================================================================================================ exporter
+
+
+@threestudio.register("mesh-exporter")
+class MeshExporter(Exporter):
+    """threestudio's `mesh-exporter` (what `launch.py --export` builds from the system's default `exporter_type`) for this
+    package's geometry and material: the atlas of uvatlas.py and the texture bake of texbake.py instead of xatlas,
+    nvdiffrast and cv2.inpaint.  Returns one ExporterOutput that the host's `save_obj` writes unchanged."""
+
+    @dataclass
+    class Config(Exporter.Config):
+        # models/exporters/mesh_exporter.py of the reference (not vendored here), restated field for field
+        fmt: str = "obj-mtl"
+        save_name: str = "model"
+        save_normal: bool = False
+        save_uv: bool = True
+        save_texture: bool = True
+        texture_size: int = 1024
+        texture_format: str = "jpg"
+        xatlas_chart_options: dict = field(default_factory=dict)
+        xatlas_pack_options: dict = field(default_factory=dict)
+        context_type: str = "gl"      # no rasteriser context is needed here; accepted and ignored
+
+    cfg: Config
+
+    def configure(self, geometry, material, background) -> None:
+        super().configure(geometry, material, background)
+        c = self.cfg
+        if c.fmt not in ("obj-mtl", "obj"):
+            raise ValueError(f"Unsupported mesh export format: {c.fmt}")
+        if dict(c.xatlas_chart_options):
+            raise ValueError(f"xatlas_chart_options {sorted(dict(c.xatlas_chart_options))} have no counterpart in the "
+                             "dreammat_b200 atlas (uvatlas.py)")
+        extra = sorted(set(dict(c.xatlas_pack_options)) - {"padding"})
+        if extra:
+            raise ValueError(f"xatlas_pack_options {extra} have no counterpart in the dreammat_b200 atlas; only 'padding' is read")
+        if c.save_texture and not c.save_uv:
+            raise ValueError("save_uv must be True when save_texture is True")
+        if not isinstance(geometry, DreamMatMesh) or not isinstance(material, DreamMatMaterial):
+            raise TypeError(f"mesh-exporter of dreammat_b200 exports its own geometry and material, got "
+                            f"{type(geometry).__name__} / {type(material).__name__}")
+
+    def __call__(self) -> List[ExporterOutput]:
+        c = self.cfg
+        geo, mat = self.geometry.impl, self.material.impl
+        mesh = _T.ExportedMesh(v_pos=geo.v_pos, t_pos_idx=geo.t_pos_idx, v_nrm=geo.v_nrm if c.save_normal else None)
+        params = {"mesh": mesh, "save_mat": c.fmt == "obj-mtl", "save_normal": c.save_normal, "save_uv": c.save_uv,
+                  "save_vertex_color": False, "map_Kd": None, "map_Ks": None, "map_Bump": None, "map_Pm": None, "map_Pr": None,
+                  "map_format": c.texture_format}
+        padding = int(dict(c.xatlas_pack_options).get("padding", 2))
+        if c.fmt == "obj-mtl" and c.save_texture:
+            baked = _T.bake_textures(geo, mat, c.texture_size, padding)
+            mesh.v_tex, mesh.t_tex_idx = baked["v_tex"], baked["t_tex_idx"]
+            params.update(map_Kd=baked["map_Kd"], map_Pm=baked["map_Pm"], map_Pr=baked["map_Pr"])
+        elif c.save_uv:
+            from .uvatlas import build_atlas
+            atlas = build_atlas(geo.v_pos.numpy(), geo.t_pos_idx.numpy(), c.texture_size, padding)
+            mesh.v_tex, mesh.t_tex_idx = torch.from_numpy(atlas.v_tex), torch.from_numpy(atlas.t_tex_idx)
+        if c.fmt == "obj" and c.save_texture:
+            mesh.v_rgb = _T.vertex_material(geo, mat)[:, :3].cpu()         # per-vertex albedo
+            params["save_vertex_color"] = True
+        return [ExporterOutput(save_name=f"{c.save_name}.obj", save_type="obj", params=params)]

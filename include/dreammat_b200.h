@@ -316,6 +316,31 @@ int dm_attention(int bf16, const void* q, int64_t ldq, int64_t q_batch_stride, c
                  int64_t ldkv, int64_t kv_batch_stride, void* out, int64_t ldo, int64_t out_batch_stride, int batch,
                  int heads, int Nq, int Nk, int head_dim, float scale, void* stream);
 
+/* ------------------------------------------------------------------ texture bake of the mesh exporter (N5)
+ * Replaces the texture half of threestudio's `mesh-exporter` (models/exporters/mesh_exporter.py: nvdiffrast UV
+ * rasterisation, per-texel geometry/material export, cv2.inpaint seam padding).  The UV atlas comes from
+ * dreammat_b200/uvatlas.py.  T (texture size) must lie in [16, 8192].  Init-time entry points; bit-reproducible.
+ * dm_uv_raster: uv_fixed [Vt,2] int32 texel coordinates with 8 sub-texel bits, tri_uv [F,3]; texel (r,c) has its centre at
+ *   (256c+128, 256r+128).  int64 edge functions + top-left rule; faces whose snapped area is <= 0 cover nothing.  The
+ *   caller guarantees that no texel centre is covered twice (the atlas is checked for it).
+ *   owner [T*T] face id or -1; bary [T*T,3] fp32 barycentrics; mask [T*T] 1 where covered. */
+int dm_uv_raster(const int32_t* uv_fixed, const int32_t* tri_uv, int64_t n_faces, int T, int32_t* owner, float* bary,
+                 uint8_t* mask, void* stream);
+/* points[i] = sum_k bary[texels[i],k] * v_pos[t_pos_idx[owner[texels[i]], k]]  (texels: from dm_compact_mask of mask) */
+int dm_texel_positions(const int32_t* texels, int64_t n, const int32_t* owner, const float* bary, const float* v_pos,
+                       const int32_t* t_pos_idx, float* points, void* stream);
+/* DreamMatMaterial.export (dreammat_material.py:765-797) of features [n,5]: sigmoid; metallic range; roughness
+ * sqrt(m*(max-min)+min+1e-7) with cfg->min_roughness / max_roughness holding the SQUARED-roughness range.
+ * out [n,5] (albedo rgb, metallic, roughness; may be NULL); texels (may be NULL): scatter (uint8)(x*255) into
+ * map_kd [T*T,3], map_pm [T*T], map_pr [T*T] at texels[i]. */
+int dm_material_export(const dm_material_cfg* cfg, const float* features, int64_t n, float* out, const int32_t* texels,
+                       uint8_t* map_kd, uint8_t* map_pm, uint8_t* map_pr, void* stream);
+/* seam fill: every texel takes the uint8 value of a covered texel at the exact minimal Euclidean distance (Meijster
+ * EDT, integer arithmetic, deterministic ties) and is written as k/255 fp32: kd_out [T*T,3], pm_out / pr_out [T*T].
+ * src [T*T] receives the source texel (r*T+c; itself where covered); scratch: 4*T*T int32. */
+int dm_seam_fill(const uint8_t* mask, int T, const uint8_t* map_kd, const uint8_t* map_pm, const uint8_t* map_pr,
+                 int32_t* scratch, int32_t* src, float* kd_out, float* pm_out, float* pr_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
